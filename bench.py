@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- rays/s (fwd+bwd) of the volumetric render hot path on BASELINE.json's config 2.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--res 1024] [--scene lego|dense]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--res 1024] [--scene lego|dense] [--dump-outputs DIR]
 
 One "step" = one pass of the hot path over one 1024x1024 frame of synthetic rays:
     Pipeline(NeuralRadianceField(HashGrid L=16,F=2,T=2^19; decoders 32-64-16 / 42-64-64-3), PackedRFTracer('ray', 2048))
@@ -55,6 +55,9 @@ def parse():
                     help="BASELINE.json config: 1 = HashGrid 8-level, 1-layer-32 MLP, 256^2 single view (the reference's CPU-runnable case; same runner as 2), "
                          "2 = HashGrid NeRF fwd+bwd (headline), 3 = nglod OctreeGrid SDF sphere trace, 4 = TriplanarGrid NeRF")
     ap.add_argument("--hidden-dim", type=int, default=0, help="configs 1/2: decoder width override (128 = the reference's best published app/nerf setting)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step computed (its outputs and the parameters it updated) as DIR/<name>.npy, "
+                         f"float32 or float64, at most {DUMP_LIMIT // 10**6} MB in all, to compare two builds on the same inputs")
     a = ap.parse_args()
     if a.config == 1 and a.res == 1024:
         a.res = 256
@@ -91,6 +94,35 @@ def workload_config(args):
             "l2": "per-step working set (hit masks + sample records, >1 GB) exceeds the 126 MB L2; a different camera every step",
             "parallelism": (f"dp{args.gpus}: {args.gpus} views per step, every rank renders rows rank::{args.gpus} of each view (same sample load on "
                             f"every rank), NCCL all-reduce of gradients") if args.gpus > 1 else "single GPU"}
+
+
+DUMP_LIMIT = 64_000_000          # bytes of array data written by --dump-outputs
+
+
+def dump_outputs(path, arrays, limit=DUMP_LIMIT):
+    """Write each array as <path>/<name>.npy, float64 where it was computed so and float32 otherwise.  The limit is shared out from
+    the smallest array up; an array larger than its share is replaced by a fixed, seeded sample of its rows, and the indices of
+    those rows are written beside it as <name>.rows.npy."""
+    os.makedirs(path, exist_ok=True)
+    arrays = {k: np.asarray(v) for k, v in arrays.items()}
+    arrays = {k: np.ascontiguousarray(v, dtype=np.float64 if v.dtype == np.float64 else np.float32) for k, v in arrays.items()}
+    left = limit
+    for i, (name, a) in enumerate(sorted(arrays.items(), key=lambda kv: (kv[1].nbytes, kv[0]))):
+        share = left // (len(arrays) - i)
+        if a.nbytes > share:
+            row_bytes = a.nbytes // a.shape[0]
+            rows = np.sort(np.random.default_rng(0).choice(a.shape[0], share // (row_bytes + 8), replace=False))
+            np.save(os.path.join(path, name + ".rows.npy"), rows.astype(np.float64))
+            a = a[rows]
+            left -= rows.size * 8
+        np.save(os.path.join(path, name + ".npy"), a)
+        left -= a.nbytes
+
+
+def host_arrays(named):
+    """name -> host copy of each tensor, float64 kept, everything else as float32 (bool masks become 0 / 1)."""
+    import torch
+    return {k: (v.detach() if v.dtype == torch.float64 else v.detach().float()).cpu().numpy() for k, v in named.items()}
 
 
 def orbit_origin(i: int):
@@ -147,10 +179,12 @@ def run_reference(args):
     nrays = args.cpu_sample_rays or 65536
     for i in range(args.warmup):              # warm-up at the timed size (page-faults of the 42 MB gradient table, thread pool spin-up)
         cpu_time_step(O, onef, spc, args, nrays, i, i)
-    times, samples = [], 0
+    times, samples, last = [], 0, {}
     for i in range(args.steps):
-        dt, ns = cpu_time_step(O, onef, spc, args, nrays, args.warmup + i, args.warmup + i)
+        dt, ns = cpu_time_step(O, onef, spc, args, nrays, args.warmup + i, args.warmup + i, keep=last)
         times.append(dt); samples += ns
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, last["st"])
     med = float(np.median(times))             # median of the steps: robust against a noisy neighbour on the shared host
     value = nrays / med
     sample = (f"{nrays} rays strided over the {args.res}^2 frame per step, full config (n={args.num_steps}); "
@@ -278,6 +312,7 @@ def run_ours(args):
         return 1000 + i * world + rank
 
     host_trace = []                        # --trace-host: wall-clock of the host-side phases of every step (diagnostics only)
+    last_rgb = [None]                      # --dump-outputs, autograd step: the image of the latest step
 
     def step(i, origins, dirs, target, nxt=None, nxt_ready=None):
         import time
@@ -297,6 +332,8 @@ def run_ours(args):
         opt.zero_grad(set_to_none=True)      # autograd then adopts the returned gradient buffers: no zero-fill + accumulate pass over the 42 MB table
         tracer.seed = seed_of(i)
         rb = pipe(rays=W.Rays(origins, dirs, dist_min=NEAR, dist_max=FAR), lod_idx=None, channels=["rgb"])
+        if args.dump_outputs:
+            last_rgb[0] = rb.rgb.detach()
         t2 = time.perf_counter()
         loss = torch.nn.functional.smooth_l1_loss(rb.rgb, target, reduction='none').mean()       # multiview_trainer.py:144-154
         t3 = time.perf_counter()
@@ -346,11 +383,14 @@ def run_ours(args):
     total_samples = 0
     for k in range(args.steps):
         i = args.warmup + k
-        step(i, *dev_rays[i], dev_tgt[i], nxt=dev_rays[i + 1] if k + 1 < args.steps else None)
+        loss = step(i, *dev_rays[i], dev_tgt[i], nxt=dev_rays[i + 1] if k + 1 < args.steps else None)
         total_samples += tracer.get_prev_num_samples()
         step_ev[k + 1].record()
     e1.record()
     barrier()
+    dumped = None
+    if args.dump_outputs and rank == 0:   # before the e2e leg below takes further optimiser steps
+        dumped = host_arrays({"loss": loss, "rgb": stepper.last_rgb if native else last_rgb[0], **dict(nef.named_parameters())})
     ms = e0.elapsed_time(e1)
     step_ms = [step_ev[k].elapsed_time(step_ev[k + 1]) for k in range(args.steps)]
     dev_allocs = torch.cuda.memory_stats(dev).get("num_device_alloc", 0) - dev_allocs0
@@ -506,6 +546,8 @@ def run_ours(args):
         print("step, premarch ms, zero_grad+forward ms, loss ms, backward ms, reduce+opt ms, cudaMallocs so far", file=sys.stderr)
         for row in host_trace:
             print(row, file=sys.stderr)
+    if dumped is not None:
+        dump_outputs(args.dump_outputs, dumped)
     print(json.dumps(line), flush=True)
     if world > 1:
         dist.destroy_process_group()
@@ -690,6 +732,8 @@ def run_config3(args):
                 print("step", k, "device allocs", ms_.get("num_device_alloc", 0), "reserved MB", ms_.get("reserved_bytes.all.current", 0) / 1e6, file=sys.stderr)
         e1.record()
         barrier()
+        if args.dump_outputs and rank == 0:
+            dump_outputs(args.dump_outputs, host_arrays({c: getattr(rb, c) for c in chans}))
         step_ms3 = [sev[k].elapsed_time(sev[k + 1]) for k in range(args.steps)]
         dev_allocs3 = torch.cuda.memory_stats(dev).get("num_device_alloc", 0) - dev_allocs0
         launches = W._cabi.launch_count() - l0
@@ -805,10 +849,14 @@ def run_config4(args):
             print(json.dumps({"parity_failure": parity}), file=sys.stderr, flush=True)
             raise SystemExit("bench.py --config 4: fused path differs from the unfused route beyond the stated tolerance")
 
+    last_rgb = [None]                      # --dump-outputs: the image of the latest step
+
     def step(i, o, d, t):
         opt.zero_grad(set_to_none=True)
         tracer.seed = 1000 + i * world + rank
         rb = pipe(rays=W.Rays(o, d, dist_min=NEAR, dist_max=FAR), channels=["rgb"])
+        if args.dump_outputs:
+            last_rgb[0] = rb.rgb.detach()
         loss = torch.nn.functional.smooth_l1_loss(rb.rgb, t, reduction='none').mean()
         loss.backward()
         reducer.reduce()
@@ -832,9 +880,11 @@ def run_config4(args):
     S_total = 0
     e0.record()
     for k in range(args.steps):
-        step(args.warmup + k, *devb[args.warmup + k]); S_total += tracer.get_prev_num_samples()
+        loss = step(args.warmup + k, *devb[args.warmup + k]); S_total += tracer.get_prev_num_samples()
     e1.record()
     barrier()
+    if args.dump_outputs and rank == 0:   # before the e2e leg below takes further optimiser steps
+        dump_outputs(args.dump_outputs, host_arrays({"loss": loss, "rgb": last_rgb[0], **dict(nef.named_parameters())}))
     launches = W._cabi.launch_count() - l0
     prof, W.ops.PROFILE = W.ops.PROFILE, None
     ms = e0.elapsed_time(e1)

@@ -1,28 +1,17 @@
-"""GPU tests (-m gpu) against the REFERENCE's OWN CUDA kernels, compiled from /root/reference/wisp/csrc into
-oracle/_ref/libwisp_ref_kernels.so by oracle/ref_kernels/build_ref.py (build container; the library travels to the GPU box):
+"""GPU tests (-m gpu) against what the ORIGINAL kaolin-wisp CUDA operators returned on the same inputs:
     hashgrid_interpolate_cuda / _backward_cuda  (A14)      uniform_sample_cuda  (A8)      find_depth_bound_cuda  (B1)
-This pins those three operators on the B200 to the code they replace, not to a restatement of it.  Skipped when the library is absent
-(a checkout that never ran the build recipe)."""
-import ctypes as C
+The outputs are stored under tests/golden/ref_*.npz by oracle/ref_kernels/golden.py (run on a B200 against the operators built from the
+original sources); the inputs are rebuilt here by the same functions.  This pins those three operators to the code they replace, not
+to a restatement of it."""
 import os
 
 import numpy as np
 import pytest
 import torch
 
+from oracle.ref_kernels import golden as G
+
 pytestmark = pytest.mark.gpu
-
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF_LIB = os.path.join(ROOT, "oracle", "_ref", "libwisp_ref_kernels.so")
-
-
-@pytest.fixture(scope="module")
-def ref():
-    if not os.path.exists(REF_LIB):
-        pytest.skip("oracle/_ref/libwisp_ref_kernels.so not built (python oracle/ref_kernels/build_ref.py in the build container)")
-    L = C.CDLL(REF_LIB)
-    L.ref_last_error.restype = C.c_char_p
-    return L
 
 
 @pytest.fixture(scope="module")
@@ -33,79 +22,52 @@ def W():
     return wisp_b200
 
 
-def _p(t):
-    return C.c_void_p(t.data_ptr())
+def _golden(name):
+    path = G.golden_path(name)
+    assert os.path.exists(path), f"{path} missing (python -m oracle.ref_kernels.golden regenerates it)"
+    return dict(np.load(path))
 
 
-def _chk(L, rc):
-    assert rc == 0, L.ref_last_error().decode()
-
-
-@pytest.mark.parametrize("F", [2, 4])
-def test_hashgrid_kernels_vs_reference_cuda(W, ref, F):
+@pytest.mark.parametrize("F", G.HASHGRID_FEATURE_DIMS)
+def test_hashgrid_kernels_vs_reference_cuda(W, F):
     """wb_hashgrid_fwd / _bwd (one launch, all LODs) vs wisp._C.ops.hashgrid_interpolate_cuda / _backward_cuda (one launch per LOD):
     dense and hashed levels, points on cell faces and at the +-1 borders.  Forward: same arithmetic -> 2 ulp-level agreement;
     backward: same products, different atomic order."""
-    torch.manual_seed(0)
-    blas = W.OctreeAS.make_dense(3, device="cuda")
-    grid = W.HashGrid.from_geometric(blas, feature_dim=F, num_lods=12, multiscale_type='cat', feature_std=1.0, codebook_bitwidth=14,
-                                     min_grid_res=8, max_grid_res=300).cuda()
-    N = 200_000
-    coords = (torch.rand(N, 3, device="cuda") * 2 - 1)
-    coords[:1000] = torch.round(coords[:1000] * 8) / 8                    # exact cell faces of the coarse levels
-    coords[1000:1100] = torch.sign(coords[1000:1100])                     # corners / borders of the unit cube
-    table = grid.codebook.feats.detach().contiguous()
-    L_, bw = len(grid.resolutions), grid.codebook_bitwidth
-    first = grid.codebook.begin_idxes.to("cuda").contiguous()
-    res_host = (C.c_int64 * L_)(*grid.resolutions)
-    ref_feats = torch.empty(N, L_ * F, device="cuda")
-    _chk(ref, ref.ref_hashgrid_fwd(0, _p(coords), C.c_int64(N), _p(table), C.c_int64(table.shape[0]), F, _p(first), L_, res_host, bw, _p(ref_feats)))
-    mine = W.ops.hashgrid(coords, bw, L_ - 1, grid.codebook)
-    err = float((mine - ref_feats).abs().max())
-    assert err <= 2e-6 * float(ref_feats.abs().max()), err
-    go = torch.randn(N, L_ * F, device="cuda")
-    ref_gt = torch.zeros_like(table)
-    _chk(ref, ref.ref_hashgrid_bwd(0, _p(coords), C.c_int64(N), _p(go), _p(table), C.c_int64(table.shape[0]), F, _p(first), L_, res_host, bw, _p(ref_gt)))
+    g = _golden(f"hashgrid_f{F}")
+    grid, coords, go, feat_rows, table_rows = G.hashgrid_case(W, F)
+    assert np.array_equal(feat_rows, g["feat_rows"]) and np.array_equal(table_rows, g["table_rows"])
+    mine = W.ops.hashgrid(coords, grid.codebook_bitwidth, len(grid.resolutions) - 1, grid.codebook)
+    assert abs(float(mine.abs().max()) - float(g["feats_absmax"])) <= 2e-6 * float(g["feats_absmax"])
+    err = float(np.abs(mine[torch.from_numpy(feat_rows).cuda()].detach().cpu().numpy() - g["feats"]).max())
+    assert err <= 2e-6 * float(g["feats_absmax"]), err
     grid.codebook.feats.grad = None
     mine.backward(go)
-    gerr = float((grid.codebook.feats.grad - ref_gt).abs().max())
-    assert gerr <= 2e-5 * float(ref_gt.abs().max()), gerr
+    gt = grid.codebook.feats.grad
+    assert abs(float(gt.abs().max()) - float(g["grad_absmax"])) <= 2e-5 * float(g["grad_absmax"])
+    gerr = float(np.abs(gt[torch.from_numpy(table_rows).cuda()].cpu().numpy() - g["grad_table"]).max())
+    assert gerr <= 2e-5 * float(g["grad_absmax"]), gerr
 
 
-def test_uniform_sampler_vs_reference_cuda(W, ref):
+def test_uniform_sampler_vs_reference_cuda(W):
     """OctreeAS._raymarch_uniform: wb_raymarch_uniform_{count,fill} vs the reference's uniform_sample_cuda kernel fed as
-    octree_as.py:340-357 feeds it (zero-count nuggets filtered, inclusive sum): ridx, depth samples and boundary bit-exact."""
-    from oracle import oracle as O
-    blas = W.OctreeAS.from_quantized_points(torch.from_numpy(O.lego_like_points(6)).cuda(), 6)
-    o, d = O.look_at_rays([-3.0, 0.65, -3.0], [0, 0, 0], 96, 96, 30.0)
-    rays = W.Rays(torch.from_numpy(o).cuda(), torch.from_numpy(d).cuda(), 0.0, 10.0)
-    n = 256
-    mr = blas.raymarch(rays, 'uniform', n, 6)
-    rt = blas.raytrace(rays, 6, with_exit=True)
-    scale = W.ops.uniform_scale(n)
-    depth = rt.depth.contiguous()
-    cnt = (torch.ceil(scale * depth[:, 1]) - torch.ceil(scale * depth[:, 0])).int()          # octree_as.py:343-345
-    nz = cnt > 0
-    ridx_f, depth_f = rt.ridx[nz].contiguous(), depth[nz].contiguous()
-    insum = torch.cumsum(cnt[nz], 0).int().contiguous()
-    V, total = int(ridx_f.shape[0]), int(insum[-1])
-    assert total == mr.ridx.shape[0] > 1000
-    r_ridx = torch.empty(total, dtype=torch.int64, device="cuda"); r_depth = torch.empty(total, device="cuda"); r_b = torch.empty(total, dtype=torch.bool, device="cuda")
-    _chk(ref, ref.ref_uniform_sample(0, scale, _p(ridx_f), _p(depth_f), _p(insum), C.c_int64(V), C.c_int64(total), _p(r_ridx), _p(r_depth), _p(r_b)))
-    assert torch.equal(mr.ridx, r_ridx) and torch.equal(mr.depth_samples[:, 0], r_depth) and torch.equal(mr.boundary, r_b)
+    octree_as.py:340-357 feeds it: ridx, depth samples and boundary bit-exact (a stored sample, then the digest of every entry)."""
+    g = _golden("uniform_sample")
+    mr, _, (_, _, insum) = G.uniform_case(W)
+    total = int(g["total"])
+    assert int(insum[-1]) == total == mr.ridx.shape[0] > 1000
+    idx = torch.from_numpy(G.sample_index(total)).cuda()
+    depth = mr.depth_samples[:, 0]
+    assert np.array_equal(mr.ridx[idx].cpu().numpy(), g["ridx"])
+    assert np.array_equal(depth[idx].cpu().numpy(), g["depth"])
+    assert np.array_equal(mr.boundary[idx].cpu().numpy(), g["boundary"])
+    assert mr.ridx.dtype == torch.int64 and mr.boundary.dtype == torch.bool
+    assert G.digest(mr.ridx) == str(g["ridx_sha256"])
+    assert G.digest(depth) == str(g["depth_sha256"])
+    assert G.digest(mr.boundary) == str(g["boundary_sha256"])
 
 
-def test_find_depth_bound_vs_reference_cuda(W, ref):
+def test_find_depth_bound_vs_reference_cuda(W):
     """wb_find_depth_bound vs find_depth_bound_cuda (cursor kernel of the SDF tracer), quirks included."""
-    rng = np.random.default_rng(3)
-    P = 5000
-    counts = rng.integers(1, 6, P); offs = np.concatenate([[0], np.cumsum(counts)]).astype(np.int32)
-    Ng = int(offs[-1])
-    en = np.sort(rng.random(Ng) * 5).astype(np.float32); depth = np.stack([en, en + 0.01 + rng.random(Ng).astype(np.float32) * 0.05], -1).astype(np.float32)
-    curr = offs[:-1].copy(); curr[::13] = -1
-    q = (rng.random(P) * 5).astype(np.float32)
-    tq, tc, td = torch.from_numpy(q).cuda(), torch.from_numpy(curr).cuda(), torch.from_numpy(depth).cuda()
-    out_ref = torch.empty(P, dtype=torch.int32, device="cuda")
-    _chk(ref, ref.ref_find_depth_bound(0, _p(tq), _p(tc), _p(td), C.c_int64(P), C.c_int64(Ng), _p(out_ref)))
-    mine = W.ops.find_depth_bound(tq[:, None], td, curr_idxes=tc)
-    assert torch.equal(mine, out_ref)
+    q, curr, depth = G.depth_bound_case()
+    mine = W.ops.find_depth_bound(q[:, None], depth, curr_idxes=curr)
+    assert np.array_equal(mine.cpu().numpy(), _golden("find_depth_bound")["out"])
