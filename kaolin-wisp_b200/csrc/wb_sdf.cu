@@ -358,8 +358,10 @@ __device__ __forceinline__ void sdf_write_hit(const WbSdfTrace& T, int64_t p, in
     T.o_depth[r] = T.S.t[p]; T.o_hit[r] = 1; T.o_alpha[r] = 1.0f;
 }
 
-template <int FT, int PT, int MINB = 2>      // MINB: resident CTAs per SM the register allocation is bounded for (threads in flight = packs handled at once)
-__global__ void __launch_bounds__(WB_SDF_THREADS, MINB)
+// register allocation bounded for 2 resident CTAs per SM (threads in flight = packs handled at once): 0.97 ms measured against
+// 1.14 / 1.31 / 1.56 ms for 1 / 3 / 4 (profiles/README.md)
+template <int FT, int PT>
+__global__ void __launch_bounds__(WB_SDF_THREADS, 2)
 wb_sdf_trace_kernel(WbOct oc, WbSdf m, WbSdfTrace T)
 {
     extern __shared__ __align__(16) float sw[];
@@ -518,10 +520,7 @@ extern "C" int wb_sdf_trace(const wb_octree* oct, const wb_sdf_desc* nef, int32_
     cudaStream_t st = (cudaStream_t)s;
     rc = sdf_scan_packs(T, num_steps, st); if (rc) return rc;
     const int smem = m.smem_floats * 4;
-    static const int want_ctas = [] { const char* v = getenv("WB_SDF_CTAS"); return v && *v ? atoi(v) : 2; }();
-    const void* kern = !sdf_fast_shape(m) ? (const void*)wb_sdf_trace_kernel<0, 0>
-                     : want_ctas >= 4 ? (const void*)wb_sdf_trace_kernel<16, 1, 4> : want_ctas == 3 ? (const void*)wb_sdf_trace_kernel<16, 1, 3>
-                     : want_ctas == 1 ? (const void*)wb_sdf_trace_kernel<16, 1, 1> : (const void*)wb_sdf_trace_kernel<16, 1, 2>;
+    const void* kern = sdf_fast_shape(m) ? (const void*)wb_sdf_trace_kernel<16, 1> : (const void*)wb_sdf_trace_kernel<0, 0>;
     if (smem > 48 * 1024) WB_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
     int per_sm = 0;
     WB_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, WB_SDF_THREADS, smem));

@@ -9,18 +9,18 @@
 // wb_tc.cuh) -> fence -> group barrier -> two elected issuer threads launch the round's UMMA chains from a shared-memory issue
 // table (A = sample tile, B = TMA-staged weight pack, D in TMEM; the bias is an init UMMA Ones x Bias^T) and commit to the
 // group's mbarrier -> the group waits, tcgen05.ld's its accumulator columns, applies the activation, writes the next tile.
-// Groups are independent (own named barrier, own mbarrier, own TMEM columns): the forward runs 3 one-group CTAs per SM, the
-// backward one two-group CTA per SM.
+// Groups are independent (own named barrier, own mbarrier, own TMEM columns): the forward runs up to 3 one-group CTAs per SM, the
+// backward one CTA of two groups (below) or of three / one wide group (wb_shade_tc_bwd3.cuh, the app/nerf decoder shape) per SM.
 //
 // Forward  (wb_shade_fwd_tc_kernel): gather 15 LODs x 8 corners (fp32 blend) -> decoders -> (r,g,b,sigma).  It also saves
 //   the gathered feature rows (fp16, chunk-major [Kp0/8][S] x 16 B: coalesced both ways) for the backward.
-// Backward (wb_mlp_bwd_tc_kernel): reloads those rows -- it touches neither the hash table nor the octree -- recomputes the
-//   decoders (tiles stay in shared memory) and per layer issues
+// Backward (wb_mlp_bwd_tc_kernel here, wb_mlp_bwd3_tc_kernel in wb_shade_tc_bwd3.cuh): reloads those rows -- it touches neither the
+//   hash table nor the octree -- recomputes the decoders (tiles stay in shared memory) and per layer issues
 //     weight grad   acc_l[in, out] += X_l^T . dY_l   (both operands MN-major straight from the sample tiles; accumulators
 //                                                     stay in TMEM for the whole kernel; a constant-one slab behind every
 //                                                     X_l tile makes row `Kp_l` the bias gradient)
 //     data grad     dX_l = dY_l . W_l                (weight pack read MN-major: no transposed copy)
-//   and writes dL/dfeat as fp16 level-major planes [L][S][F].
+//   and writes dL/dfeat as fp16 level-major planes [L][S][F] (the three-group kernel scatters them itself on F == 2 'cat' hash grids).
 // Scatter  (wb_table_scatter_kernel, SIMT): lanes = consecutive samples; a thread builds its sample position once and walks all
 //   LODs; per LOD, runs of lanes that fall into the same cell are summed with a segmented warp scan and only the last lane of a
 //   run issues the reductions (x-neighbour entries that differ only in bit 0 as one 16-byte red.global.add.v4.f32).
@@ -641,54 +641,7 @@ __device__ __forceinline__ void tile_gather_ta(const WbGrid& g, uint32_t arow, i
     tc_st_wait();
 }
 
-// Software-pipelined form of tile_gather_ta (WB_TC_FWD_PIPE=1): the eight corner loads of LOD k are issued, THEN the cell / index /
-// coefficient arithmetic of LOD k+1 runs (~200 instructions), and only then are LOD k's corners blended -- the gather's L1/L2 latency
-// (long_scoreboard: 5.2 stalls per issue, profiles/r02e) overlaps ALU work of the same warp.  Needs more registers than the plain form.
-__device__ __forceinline__ void tile_gather_ta_pipe(const WbGrid& g, uint32_t arow, int half, float px, float py, float pz,
-                                                    uint4* __restrict__ save, int64_t S, int64_t s, bool valid)
-{
-    const int nlev = min(g.L, g.lod_idx);                        // LODs >= lod_idx are zeroed (hash_grid.py:226-229)
-    uint32_t idx[8]; float cf[8]; float2 c[8];
-    int lnext = 4 * half;
-    bool have = false;
-    if (lnext < nlev) {
-        wb_corner_setup(g, lnext, px, py, pz, idx, cf);
-        const float2* tb = reinterpret_cast<const float2*>(g.table + g.begin[lnext] * 2);
-#pragma unroll
-        for (int j = 0; j < 8; ++j) c[j] = __ldg(tb + idx[j]);
-        have = true;
-    }
-    for (int l0 = 4 * half; l0 < g.L; l0 += 8) {
-        float v[8];
-#pragma unroll
-        for (int q = 0; q < 4; ++q) {
-            const int l = l0 + q;
-            if (l >= nlev || !have) { v[2 * q] = 0.0f; v[2 * q + 1] = 0.0f; continue; }
-            float cfl[8];
-#pragma unroll
-            for (int j = 0; j < 8; ++j) cfl[j] = cf[j];
-            const int ln = ((l & 3) == 3) ? l + 5 : l + 1;         // this thread's next LOD: 4h, 4h+1, 4h+2, 4h+3, 4h+8, ...
-            const bool more = ln < nlev;
-            if (more) wb_corner_setup(g, ln, px, py, pz, idx, cf);
-            float a0 = c[0].x * cfl[0], a1 = c[0].y * cfl[0];
-#pragma unroll
-            for (int j = 1; j < 8; ++j) { a0 = fmaf(c[j].x, cfl[j], a0); a1 = fmaf(c[j].y, cfl[j], a1); }
-            v[2 * q] = a0; v[2 * q + 1] = a1;
-            if (more) {
-                const float2* tb = reinterpret_cast<const float2*>(g.table + g.begin[ln] * 2);
-#pragma unroll
-                for (int j = 0; j < 8; ++j) c[j] = __ldg(tb + idx[j]);
-            }
-            have = more;
-        }
-        uint4 qv; qv.x = tc_pack2(v[0], v[1]); qv.y = tc_pack2(v[2], v[3]); qv.z = tc_pack2(v[4], v[5]); qv.w = tc_pack2(v[6], v[7]);
-        tc_st4(arow + (uint32_t)(l0 >> 2) * 4u, qv);
-        if (save != nullptr && valid) save[(int64_t)(l0 >> 2) * S + s] = qv;
-    }
-    tc_st_wait();
-}
-
-template <int MINB, bool TA, bool GX = false, bool PIPE = false>   // MINB: resident CTAs per SM the register allocation is bounded for; TA: activations in tensor
+template <int MINB, bool TA, bool GX = false>   // MINB: resident CTAs per SM the register allocation is bounded for; TA: activations in tensor
                                                 // memory; GX: triplanar / octree feature grid (wb_featx.cuh) instead of the hash grid
 __global__ void __launch_bounds__(TC_GROUP, MINB)
 wb_shade_fwd_tc_kernel(WbGrid g, WbGridX gx, WbTc m, const uint8_t* __restrict__ blob, TcIn in, float4* __restrict__ shaded)
@@ -724,8 +677,7 @@ wb_shade_fwd_tc_kernel(WbGrid g, WbGridX gx, WbTc m, const uint8_t* __restrict__
         const float pz = wb_addcmul(__ldg(in.origins + 3 * ray + 2), __ldg(in.dirs + 3 * ray + 2), t);
         // density-decoder input row: grid features (+ position embedding), zero padded to Kp; the two threads of a row split the LODs
         if (TA) {
-            if (PIPE) tile_gather_ta_pipe(g, c.tmem + ((uint32_t)c.laneq << 16) + (uint32_t)m.work_col[1], c.h, px, py, pz, in.x0_save, in.S, s, valid);
-            else tile_gather_ta(g, c.tmem + ((uint32_t)c.laneq << 16) + (uint32_t)m.work_col[1], c.h, px, py, pz, in.x0_save, in.S, s, valid);
+            tile_gather_ta(g, c.tmem + ((uint32_t)c.laneq << 16) + (uint32_t)m.work_col[1], c.h, px, py, pz, in.x0_save, in.S, s, valid);
         } else {
             if (!GX) tile_gather(g, t0, c.r, c.h, px, py, pz);
             else if (c.h == 0) {
@@ -770,32 +722,22 @@ static int tc_launch_ray_embed(const WbTc& m, const wb_rays* rays, void* workspa
     return WB_OK;
 }
 
-// Tuning knobs (defaults = the measured optimum on B200 for the app/nerf configuration, profiles/README.md); the environment
-// overrides exist for the sweeps and are read once per process.
-static int tc_env_int(const char* name, int dflt) { const char* v = getenv(name); return v && *v ? atoi(v) : dflt; }
-static int tc_knob_fuse_scatter() { static const int v = tc_env_int("WB_TC_FUSE_SCATTER", 1); return v; }     // 0 separate kernel, 1 last epilogue (default), 2 pipelined
-static int tc_knob_bwd_groups() { static const int v = tc_env_int("WB_TC_BWD_GROUPS", 3); return v; }
-static int tc_knob_fwd_tmema() { static const int v = tc_env_int("WB_TC_FWD_TMEMA", 1); return v; }
-static int tc_knob_fwd_pipe() { static const int v = tc_env_int("WB_TC_FWD_PIPE", 0); return v; }
-static int tc_knob_fwd_ctas() { static const int v = tc_env_int("WB_TC_FWD_CTAS", 3); return v; }
-static int tc_knob_fuse_scatter_wide() { static const int v = tc_env_int("WB_TC_FUSE_SCATTER_WIDE", 0); return v; }
-static int64_t tc_knob_wide_min_s() { static const int v = tc_env_int("WB_TC_WIDE_MIN_S", 1 << 20); return v; }      // below this many samples the chunked schedule is not worth its launches
-static int tc_knob_wide_chunks() { static const int v = tc_env_int("WB_TC_WIDE_CHUNKS", 4); return v; }       // 1: no overlap of decoder backward and table scatter
-static int tc_knob_scatter_lpb() { static const int v = tc_env_int("WB_TC_SCATTER_LPB", 16); return v; }
-static int tc_knob_scatter_idx2() { static const int v = tc_env_int("WB_TC_SCATTER_IDX2", 1); return v; }
-static int tc_knob_scatter_ctas() { static const int v = tc_env_int("WB_TC_SCATTER_CTAS", 16); return v; }
-static int tc_knob_scatter_h2() { static const int v = tc_env_int("WB_TC_SCATTER_H2", 1); return v; }
-static int tc_knob_scatter_v4() { static const int v = tc_env_int("WB_TC_SCATTER_V4", 1); return v; }
+// Launch shapes: the measured optimum on B200 for the app/nerf configuration (the sweeps are in profiles/README.md)
+constexpr int TC_FWD_CTAS = 3;                 // forward CTAs per SM at most (4 measured slower: 4.26 vs 3.19 ms)
+constexpr int TC_WIDE_CHUNKS = 4;              // sample chunks of the wide-decoder backward schedule (wb_tc_shade_bwd)
+constexpr int64_t TC_WIDE_MIN_S = 1 << 20;     // below this many samples the chunked schedule is not worth its launches
+constexpr int TC_SCATTER_LPB = 16;             // LODs per CTA row of the table scatter
+constexpr int TC_SCATTER_CTAS = 16;            // table-scatter CTAs per SM
 
 int wb_tc_shade_fwd(const wb_nef_desc* nef, const float* blob, const wb_rays* rays, const float* rec_t, const int32_t* rec_ray,
                     int64_t S, float* shaded, void* feat_save, void* workspace, cudaStream_t st)
 {
     WbGrid g; int rc = wb_make_grid(nef, &g); if (rc) return rc;
     WbGridX gx; rc = wb_make_gridx(nef, false, &gx); if (rc) return rc;
-    // Default since round 2 (WB_TC_FWD_TMEMA=0 selects the shared-memory tile): activations in tensor memory, A operand read from TMEM
-    // (wb_tc.cuh tc_mma_ts); measured 3.10 -> 2.86 ms on the 1024^2 frame, same results.
-    // Applies to the specialised F == 2 'cat' gather without position embedding, whose rows are whole 16-byte chunks.
-    const bool ta = tc_knob_fwd_tmema() && nef->grid_kind == 0 && nef->feature_dim == 2 && nef->multiscale == 0 && nef->pos_mode == 0 &&
+    // Activations in tensor memory, A operand read from TMEM (wb_tc.cuh tc_mma_ts): measured 2.86 ms on the 1024^2 frame against
+    // 3.10 ms for the shared-memory tile, same results.  Applies to the specialised F == 2 'cat' gather without position embedding,
+    // whose rows are whole 16-byte chunks; every other grid keeps the shared-memory tile.
+    const bool ta = nef->grid_kind == 0 && nef->feature_dim == 2 && nef->multiscale == 0 && nef->pos_mode == 0 &&
                     (nef->num_lods * nef->feature_dim) % 16 == 0;
     WbTc m; rc = wb_tc_make(nef, false, &m, ta); if (rc) return rc;
     if (ta) {   // no activation tile in shared memory: the parameter blob and the bias tile move to the front
@@ -807,29 +749,28 @@ int wb_tc_shade_fwd(const wb_nef_desc* nef, const float* blob, const wb_rays* ra
     TcIn in = { rays->origins, rays->dirs, rec_t, rec_ray, S, reinterpret_cast<const uint4*>(workspace), reinterpret_cast<uint4*>(feat_save), nullptr };
     // CTAs per SM: each is one sub-tile group; more groups in flight hide the gather and round latencies (measured sweep in
     // profiles/README.md).  The register bound of the instantiation must match, or the hardware silently runs fewer.
-    int per_sm = (227 * 1024) / (m.smem_bytes + 4096); per_sm = max(1, min(per_sm, 512 / m.tmem_cols));
-    per_sm = max(2, min(min(per_sm, 4), tc_knob_fwd_ctas()));
-    // the generic grids keep more state per thread.  Triplanar (12 planes x 4 texel loads in flight): 3 CTAs per SM at 80 registers beat 2 at 128
-    // despite 144 B of spills (config 4 forward 105 -> 88 ms measured); the octree gather (up to 32 accumulators) stays at 2
-    if (gx.kind != 0) per_sm = max(2, min(min(per_sm, 4), tc_env_int("WB_TC_GX_CTAS", gx.kind == 1 ? 3 : 2)));
-    const bool pipe = ta && tc_knob_fwd_pipe() != 0 && per_sm <= 3;
-    auto kern = gx.kind != 0 ? (per_sm == 4 ? wb_shade_fwd_tc_kernel<4, false, true> : per_sm == 3 ? wb_shade_fwd_tc_kernel<3, false, true> : wb_shade_fwd_tc_kernel<2, false, true>)
-              : pipe ? (per_sm == 2 ? wb_shade_fwd_tc_kernel<2, true, false, true> : wb_shade_fwd_tc_kernel<3, true, false, true>)
-              : ta ? (per_sm == 2 ? wb_shade_fwd_tc_kernel<2, true> : per_sm == 3 ? wb_shade_fwd_tc_kernel<3, true> : wb_shade_fwd_tc_kernel<4, true>)
-                   : (per_sm == 2 ? wb_shade_fwd_tc_kernel<2, false> : per_sm == 3 ? wb_shade_fwd_tc_kernel<3, false> : wb_shade_fwd_tc_kernel<4, false>);
+    // The generic grids keep more state per thread.  Triplanar (12 planes x 4 texel loads in flight): 3 CTAs per SM at 80 registers beat 2
+    // at 128 despite 144 B of spills (config 4 forward 105 -> 88 ms measured); the octree gather (up to 32 accumulators) stays at 2.
+    int per_sm = (227 * 1024) / (m.smem_bytes + 4096);
+    per_sm = max(2, min(min(per_sm, 512 / m.tmem_cols), gx.kind == 2 ? 2 : TC_FWD_CTAS));
+    // [CTAs per SM - 2][shared-memory tile, TMEM-A, feature grid]
+    using FwdKernel = decltype(&wb_shade_fwd_tc_kernel<2, false>);
+    static const FwdKernel kerns[2][3] = { { wb_shade_fwd_tc_kernel<2, false>, wb_shade_fwd_tc_kernel<2, true>, wb_shade_fwd_tc_kernel<2, false, true> },
+                                           { wb_shade_fwd_tc_kernel<3, false>, wb_shade_fwd_tc_kernel<3, true>, wb_shade_fwd_tc_kernel<3, false, true> } };
+    const int variant = gx.kind != 0 ? 2 : ta ? 1 : 0;
+    const FwdKernel kern = kerns[per_sm - 2][variant];
     {   // function attributes are driver calls that can wait behind other driver work (e.g. an NVML poll): set them once, not per launch
-        static int64_t done_for[24] = { -1, -1, -1, -1, -1, -1, -1, -1, -1, -1, -1, -1, -1, -1, -1, -1, -1, -1, -1, -1, -1, -1, -1, -1 };
-        if (done_for[gx.kind != 0 ? 16 + per_sm : pipe ? 10 + per_sm : per_sm + (ta ? 5 : 0)] != WB_ATTR_KEY(m.smem_bytes)) {
+        static int64_t done_for[2][3] = { { -1, -1, -1 }, { -1, -1, -1 } };
+        if (done_for[per_sm - 2][variant] != WB_ATTR_KEY(m.smem_bytes)) {
             WB_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, m.smem_bytes));
             WB_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributePreferredSharedMemoryCarveout,
                                          min(100, (per_sm * (m.smem_bytes + 4096) * 100) / (228 * 1024) + 1)));
-            done_for[gx.kind != 0 ? 16 + per_sm : pipe ? 10 + per_sm : per_sm + (ta ? 5 : 0)] = WB_ATTR_KEY(m.smem_bytes);
+            done_for[per_sm - 2][variant] = WB_ATTR_KEY(m.smem_bytes);
         }
     }
     const int64_t ntiles = (S + TC_ROWS - 1) / TC_ROWS;
     int64_t grid = (int64_t)wb_num_sms() * per_sm; if (grid > ntiles) grid = ntiles;
-    const int xscratch = 0;
-    kern<<<(unsigned)grid, TC_GROUP, m.smem_bytes + xscratch, st>>>(g, gx, m, reinterpret_cast<const uint8_t*>(blob), in, reinterpret_cast<float4*>(shaded));
+    kern<<<(unsigned)grid, TC_GROUP, m.smem_bytes, st>>>(g, gx, m, reinterpret_cast<const uint8_t*>(blob), in, reinterpret_cast<float4*>(shaded));
     WB_LAUNCH_CHECK();
     return WB_OK;
 }
@@ -993,8 +934,8 @@ wb_mlp_bwd_tc_kernel(WbTc m, const uint8_t* __restrict__ blob, TcIn in, const fl
 // ---------------------------------------------------------------------------------------------------------------
 // table scatter: dL/dfeat planes -> hash table (hashgrid_interpolate_cuda.cu:151-160), with warp-level run merging
 // ---------------------------------------------------------------------------------------------------------------
-template <int F, bool H2, bool IDX2>   // H2: the run sums travel through the warp scan as loss-scaled fp16 pairs (one shuffle per corner)
-                                       // IDX2: corner entries through wb_corner_indices (one multiply per axis) instead of 8 x wb_hash_idx
+template <int F>   // F == 2: the run sums travel through the warp scan as loss-scaled fp16 pairs (one shuffle per corner) and the corner
+                   // entries come from wb_corner_indices (one multiply per axis); F == 0: any g.F, 8 x wb_hash_idx and fp32 run sums
 __global__ void __launch_bounds__(256)
 wb_table_scatter_kernel(WbGrid g, TcIn in, const __half* __restrict__ dfeat, int planes, int levels, int lpb,
                         const float* __restrict__ scale_p, float* __restrict__ gtable, int pair_v4)
@@ -1033,7 +974,7 @@ wb_table_scatter_kernel(WbGrid g, TcIn in, const __half* __restrict__ dfeat, int
                 const float xy00 = jx * jy, xy01 = jx * wy, xy10 = wx * jy, xy11 = wx * wy;
                 cf[0] = xy00 * jz; cf[1] = xy00 * wz; cf[2] = xy01 * jz; cf[3] = xy01 * wz;
                 cf[4] = xy10 * jz; cf[5] = xy10 * wz; cf[6] = xy11 * jz; cf[7] = xy11 * wz;
-                if (IDX2) wb_corner_indices(g, l, ix, iy, iz, idx);
+                if (F == 2) wb_corner_indices(g, l, ix, iy, iz, idx);
                 else {
 #pragma unroll
                     for (int j = 0; j < 8; ++j) idx[j] = wb_hash_idx(ix + ((j & 4) >> 2), iy + ((j & 2) >> 1), iz + (j & 1), g.res[l], g.Tmask, g.dense[l]);
@@ -1061,7 +1002,7 @@ wb_table_scatter_kernel(WbGrid g, TcIn in, const __half* __restrict__ dfeat, int
             for (int o = 16; o > 0; o >>= 1) maxd = max(maxd, __shfl_xor_sync(0xffffffffu, maxd, o));
             if (F == 2) {
                 float v0[8], v1[8];
-                if (H2 && maxd > 0) {
+                if (maxd > 0) {
                     // gradients arrive as fp16 anyway: scan the (still loss-scaled) products as half2, unscale after the scan
                     const float s0 = gv[0] * scale, s1 = gv[1] * scale;
                     __half2 h[8];
@@ -1212,7 +1153,7 @@ wb_featx_scatter_kernel(WbGridX gx, TcIn in, const __half* __restrict__ dfeat, i
     }
 }
 
-#include "wb_shade_tc_bwd3.cuh"          // three-group variant: the default for the app/nerf decoder shape (WB_TC_BWD_GROUPS=2 selects the kernel above)
+#include "wb_shade_tc_bwd3.cuh"          // three groups / one wide group: the app/nerf decoder shape; the kernel above serves the shapes it refuses
 
 // decoder backward only: dL/d(shaded) -> weight gradients + dL/dfeat planes in the workspace
 // grad_table != NULL asks for the table scatter to be fused into the decoder backward; *fused_out reports whether it was (it is for the
@@ -1244,21 +1185,22 @@ int wb_tc_decoder_bwd_ex(const wb_nef_desc* nef, const float* blob, const wb_ray
     const int64_t S_launch = (g_tc_s_end ? g_tc_s_end : S) - g_tc_s_begin;
     TcGrads G = { grad_dens, grad_col, scale, dfeat, planes, width };
     TcB3Plan plan;
-    if ((tc_knob_bwd_groups() == 3 || !m.fits2) && tc_b3_plan(m, &plan)) {     // wb_shade_tc_bwd3.cuh: three sub-tile groups per SM (4.53 -> 3.69 ms measured),
-        WbGrid g; memset(&g, 0, sizeof(g));                                     // or one 128-wide group (hidden_dim = 128)
-        const int wide = plan.groups == 1 ? 1 : 0;
+    if (tc_b3_plan(m, &plan)) {      // wb_shade_tc_bwd3.cuh: three sub-tile groups per SM (3.69 ms measured against 4.53 ms for the two-group
+        WbGrid g; memset(&g, 0, sizeof(g));    // kernel below), or one 128-wide group (hidden_dim = 128)
         // one wide group per SM: the fused scatter has only 8 warps to issue from and measured slower than the stand-alone scatter kernel
-        // (16.0 vs 13.7 ms at hidden_dim 128 on the 1024^2 frame), so it is opt-in there (WB_TC_FUSE_SCATTER_WIDE=1)
-        const bool fuse = grad_table != nullptr && tc_knob_fuse_scatter() && nef->grid_kind == 0 && nef->feature_dim == 2 && nef->multiscale == 0 &&
-                          planes <= 16 && (!wide || tc_knob_fuse_scatter_wide());
+        // (16.0 vs 13.7 ms at hidden_dim 128 on the 1024^2 frame), so only the three-group kernel fuses it
+        const bool fuse = grad_table != nullptr && nef->grid_kind == 0 && nef->feature_dim == 2 && nef->multiscale == 0 && planes <= 16 &&
+                          plan.groups == 3;
         if (fuse) { rc = wb_make_grid(nef, &g); if (rc) return rc; }
-        const int fmode = !fuse ? 0 : (tc_knob_fuse_scatter() == 2 ? 2 : (tc_knob_fuse_scatter() == 3 && !wide) ? 3 : 1);
-        auto kern3 = wide ? (fmode == 2 ? wb_mlp_bwd3_tc_kernel<2, 1> : fmode ? wb_mlp_bwd3_tc_kernel<1, 1> : wb_mlp_bwd3_tc_kernel<0, 1>)
-                          : fmode == 3 ? wb_mlp_bwd3_tc_kernel<3, 3> : fmode == 2 ? wb_mlp_bwd3_tc_kernel<2, 3> : fmode == 1 ? wb_mlp_bwd3_tc_kernel<1, 3> : wb_mlp_bwd3_tc_kernel<0, 3>;
-        static int64_t done3[2][4] = { { -1, -1, -1, -1 }, { -1, -1, -1, -1 } };
-        if (done3[wide][fmode] != WB_ATTR_KEY(plan.smem_bytes)) {
+        // [one wide group, three groups, three groups + fused scatter]
+        using Bwd3Kernel = decltype(&wb_mlp_bwd3_tc_kernel<false, 3>);
+        static const Bwd3Kernel kerns3[3] = { wb_mlp_bwd3_tc_kernel<false, 1>, wb_mlp_bwd3_tc_kernel<false, 3>, wb_mlp_bwd3_tc_kernel<true, 3> };
+        const int variant = plan.groups == 1 ? 0 : fuse ? 2 : 1;
+        const Bwd3Kernel kern3 = kerns3[variant];
+        static int64_t done3[3] = { -1, -1, -1 };
+        if (done3[variant] != WB_ATTR_KEY(plan.smem_bytes)) {
             WB_CUDA(cudaFuncSetAttribute(kern3, cudaFuncAttributeMaxDynamicSharedMemorySize, plan.smem_bytes));
-            done3[wide][fmode] = WB_ATTR_KEY(plan.smem_bytes);
+            done3[variant] = WB_ATTR_KEY(plan.smem_bytes);
         }
         const int64_t nctas3 = ((S_launch + TC_ROWS - 1) / TC_ROWS + plan.groups - 1) / plan.groups;
         int64_t grid3 = (int64_t)wb_num_sms(); if (grid3 > nctas3) grid3 = nctas3;
@@ -1305,14 +1247,11 @@ int wb_tc_table_scatter(const wb_nef_desc* nef, const wb_rays* rays, const float
     const int levels = g.multiscale == 0 ? planes : g.L;
     if (levels > 0) {
         // LODs per CTA row: the sample position / record loads are shared by `lpb` LODs (measured sweep in profiles/README.md)
-        const int lpb = max(1, min(levels, tc_knob_scatter_lpb()));
-        int64_t bx = (S_launch + 255) / 256; const int64_t cap = (int64_t)wb_num_sms() * tc_knob_scatter_ctas(); if (bx > cap) bx = cap;
+        const int lpb = max(1, min(levels, TC_SCATTER_LPB));
+        int64_t bx = (S_launch + 255) / 256; const int64_t cap = (int64_t)wb_num_sms() * TC_SCATTER_CTAS; if (bx > cap) bx = cap;
         dim3 grid2((unsigned)bx, (unsigned)((levels + lpb - 1) / lpb));
-        const int v4 = tc_knob_scatter_v4();
-        if (g.F == 2 && tc_knob_scatter_h2() && tc_knob_scatter_idx2()) wb_table_scatter_kernel<2, true, true><<<grid2, 256, 0, st>>>(g, in, dfeat, planes, levels, lpb, scale, grad_table, v4);
-        else if (g.F == 2 && tc_knob_scatter_h2()) wb_table_scatter_kernel<2, true, false><<<grid2, 256, 0, st>>>(g, in, dfeat, planes, levels, lpb, scale, grad_table, v4);
-        else if (g.F == 2) wb_table_scatter_kernel<2, false, false><<<grid2, 256, 0, st>>>(g, in, dfeat, planes, levels, lpb, scale, grad_table, v4);
-        else wb_table_scatter_kernel<0, false, false><<<grid2, 256, 0, st>>>(g, in, dfeat, planes, levels, lpb, scale, grad_table, 0);
+        auto kern = g.F == 2 ? wb_table_scatter_kernel<2> : wb_table_scatter_kernel<0>;
+        kern<<<grid2, 256, 0, st>>>(g, in, dfeat, planes, levels, lpb, scale, grad_table, g.F == 2);
         WB_LAUNCH_CHECK();
     }
     return WB_OK;
@@ -1321,7 +1260,7 @@ int wb_tc_table_scatter(const wb_nef_desc* nef, const wb_rays* rays, const float
 // Wide decoders (one 256-thread group per SM, half the register file and all the other warp slots idle): the sample range is cut
 // into chunks; the decoder backward of chunk c+1 runs on the caller's stream while the table scatter of chunk c (an issue-bound SIMT
 // kernel with 48 registers per thread and no shared memory: two of its CTAs fit beside a decoder CTA) runs on a side stream.
-struct TcSide { cudaStream_t stream; cudaEvent_t ev[17]; bool ok; };
+struct TcSide { cudaStream_t stream; cudaEvent_t ev[TC_WIDE_CHUNKS + 1]; bool ok; };
 static TcSide* tc_side_stream()
 {
     static TcSide side[64];
@@ -1329,7 +1268,7 @@ static TcSide* tc_side_stream()
     TcSide& s = side[dev];
     if (!s.ok) {
         if (cudaStreamCreateWithFlags(&s.stream, cudaStreamNonBlocking) != cudaSuccess) return nullptr;
-        for (int i = 0; i < 17; ++i) if (cudaEventCreateWithFlags(&s.ev[i], cudaEventDisableTiming) != cudaSuccess) return nullptr;
+        for (int i = 0; i <= TC_WIDE_CHUNKS; ++i) if (cudaEventCreateWithFlags(&s.ev[i], cudaEventDisableTiming) != cudaSuccess) return nullptr;
         s.ok = true;
     }
     return &s;
@@ -1341,11 +1280,10 @@ int wb_tc_shade_bwd(const wb_nef_desc* nef, const float* blob, const wb_rays* ra
 {
     {
         WbTc m; TcB3Plan plan;
-        int chunks = tc_knob_wide_chunks(); if (chunks > 16) chunks = 16;
         TcSide* side = nullptr;
-        if (chunks > 1 && S >= tc_knob_wide_min_s() && nef->grid_kind == 0 && grad_table && wb_tc_make(nef, true, &m) == WB_OK && !m.fits2 &&
-            tc_b3_plan(m, &plan) && plan.groups == 1 && !tc_knob_fuse_scatter_wide() && (side = tc_side_stream()) != nullptr) {
-            const int64_t per = ((S + chunks - 1) / chunks + TC_ROWS - 1) / TC_ROWS * TC_ROWS;
+        if (S >= TC_WIDE_MIN_S && nef->grid_kind == 0 && grad_table && wb_tc_make(nef, true, &m) == WB_OK && !m.fits2 &&
+            tc_b3_plan(m, &plan) && plan.groups == 1 && (side = tc_side_stream()) != nullptr) {
+            const int64_t per = ((S + TC_WIDE_CHUNKS - 1) / TC_WIDE_CHUNKS + TC_ROWS - 1) / TC_ROWS * TC_ROWS;
             int rc = WB_OK, c = 0;
             for (int64_t s0 = 0; s0 < S && rc == WB_OK; s0 += per, ++c) {
                 g_tc_s_begin = s0; g_tc_s_end = s0 + per < S ? s0 + per : S;
@@ -1356,7 +1294,7 @@ int wb_tc_shade_bwd(const wb_nef_desc* nef, const float* blob, const wb_rays* ra
             }
             g_tc_s_begin = 0; g_tc_s_end = 0;
             // the caller's stream continues after the last scatter (also on an error path: never leave the side stream unjoined)
-            if (cudaEventRecord(side->ev[16], side->stream) != cudaSuccess || cudaStreamWaitEvent(st, side->ev[16], 0) != cudaSuccess) { if (rc == WB_OK) rc = WB_ERR_CUDA; }
+            if (cudaEventRecord(side->ev[TC_WIDE_CHUNKS], side->stream) != cudaSuccess || cudaStreamWaitEvent(st, side->ev[TC_WIDE_CHUNKS], 0) != cudaSuccess) { if (rc == WB_OK) rc = WB_ERR_CUDA; }
             return rc;
         }
     }

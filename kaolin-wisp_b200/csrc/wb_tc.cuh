@@ -52,7 +52,7 @@ __device__ __forceinline__ uint32_t tc_elect_one()
     return pred;
 }
 // A operand read from TENSOR MEMORY (dense fp16: lane = row, two halfs per 32-bit column, K-major only), B from shared memory.
-// Used by the forward kernel (WB_TC_FWD_TMEMA, default on; see wb_shade_tc.cu): activations never touch shared memory.
+// Used by the TMEM-A forward kernel (F == 2 'cat' hash grids; see wb_shade_tc.cu): activations never touch shared memory.
 __device__ __forceinline__ void tc_mma_ts(uint32_t tmem_d, uint32_t tmem_a, uint64_t bdesc, uint32_t idesc, uint32_t accumulate)
 {
     asm volatile("{\n\t.reg .pred p;\n\tsetp.ne.b32 p, %4, 0;\n\t"
